@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the hot path's headline metric on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -41,6 +41,13 @@ max-over-ranks time.
 
 --impl reference: times the reference's CPU implementation of the same step (full-size octree
 build + a bounded query sample, extrapolated linearly) on all host threads; rank 0 only.
+
+--dump-outputs DIR: after the run, every rank saves the normals its last timed headline step
+returned for the points it owns (halo rows left out), float32, rows in the order of its own
+seeded slab: DIR/normals.npy on one GPU, DIR/normals_rank<r>.npy on N > 1.  Above
+DUMP_ROWS / N owned points a rank keeps a fixed-seed sample of that many rows
+(np.random.default_rng(0), sorted), so two builds of the library can be compared output for
+output on identical inputs.
 """
 import argparse
 import importlib
@@ -55,12 +62,29 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (which may be read-only)
 
 N_POINTS = 10_000_000
 K = 15
 HALO = 0.05
 ALGORITHMIC_BYTES_PER_NORMAL = 12 + 12 * K + 12  # SURVEY.md §8d: query + k winners + normal out
 METRIC = "normals/sec (estimate_normals k=15, 10M-pt noisy plane; index build + fused kNN->PCA per step)"
+DUMP_ROWS = 4_000_000  # 48 MB of float32 normals over all ranks: a dump stays under 64 MB
+
+
+def dump_outputs(path, normals, max_rows):
+    """Save `normals` (an (n, 3) CUDA tensor) as `path`: every row when n <= max_rows, else a
+    sorted fixed-seed sample of max_rows rows."""
+    import torch
+
+    n = normals.shape[0]
+    if n <= max_rows:
+        sample = normals
+    else:
+        rows = np.sort(np.random.default_rng(0).choice(n, max_rows, replace=False))
+        sample = normals[torch.from_numpy(rows).to(normals.device)]
+    os.makedirs(os.path.dirname(path) or ".", exist_ok=True)
+    np.save(path, sample.cpu().numpy().astype(np.float32))
 
 
 def measured_peak_gbs():
@@ -739,6 +763,11 @@ def run_ours(args):
         }
         line.update(extras)
         print(json.dumps(line))
+    if args.dump_outputs:
+        # d_nrm is untouched since the last timed step; its first n_owned rows are this rank's
+        # own points (the halo strips sit behind them)
+        name = "normals.npy" if world == 1 else "normals_rank%d.npy" % rank
+        dump_outputs(os.path.join(args.dump_outputs, name), d_nrm[:n_owned], DUMP_ROWS // world)
     if world > 1:
         dist.destroy_process_group()
     return 0
@@ -757,7 +786,15 @@ def main():
                     help="skip the extra legs (knn, radius, filter, sweep point, strong, scan100M)")
     ap.add_argument("--e2e-threads", type=int, default=4,
                     help="host threads streaming clouds through the C ABI in the e2e leg (N = 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="save the normals of the last timed step as DIR/normals.npy, one file "
+                         "per rank on N > 1 (a fixed-seed sample of %d rows over all ranks above "
+                         "that size)" % DUMP_ROWS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs saves what the GPU path computed: it needs --impl ours")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

@@ -30,7 +30,7 @@ def oracle():
 @pytest.fixture(scope="session")
 def ref():
     """The reference's own headers behind a C bridge; None when oracle/_ref was not built
-    (it can only be built where /root/reference exists and then travels with the snapshot)."""
+    (it can only be built with PCP_REFERENCE naming a checkout of the reference)."""
     from oracle_lib import RefBridge, build_oracle, have_ref
 
     build_oracle()

@@ -1,8 +1,9 @@
 """Generates tests/golden/ref_fixtures.npz by running the UNMODIFIED reference (through
-oracle/_ref/libpcp_ref.so, i.e. /root/reference/include compiled in place) on small seeded
-clouds.  Only runnable where /root/reference exists; the committed .npz is what travels.
+oracle/_ref/libpcp_ref.so, i.e. $PCP_REFERENCE/include compiled in place) on small seeded
+clouds.  Only runnable with PCP_REFERENCE naming a reference checkout; the committed .npz is
+what travels.
 
-    python tests/golden/make_fixtures.py
+    PCP_REFERENCE=<checkout> python tests/golden/make_fixtures.py
 """
 import os
 import sys

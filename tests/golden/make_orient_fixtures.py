@@ -1,8 +1,9 @@
 """Generates tests/golden/ref_orient.npz by running the UNMODIFIED reference's
 propagate_normal_orientations (oracle/_ref/libpcp_ref_orient.so) with its own kd-tree kNN on
-small seeded clouds.  Only runnable where /root/reference exists; the committed .npz travels.
+small seeded clouds.  Only runnable with PCP_REFERENCE naming a reference checkout; the
+committed .npz travels.
 
-    python tests/golden/make_orient_fixtures.py
+    PCP_REFERENCE=<checkout> python tests/golden/make_orient_fixtures.py
 """
 import os
 import sys

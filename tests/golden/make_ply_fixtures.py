@@ -1,8 +1,9 @@
 """Generates tests/golden/ref_ply.npz: the byte streams the UNMODIFIED reference writer
 (pcp::io::write_ply, through oracle/_ref/libpcp_ref_ply.so) produces for a small cloud in each
-of the three formats.  Only runnable where /root/reference exists; the .npz travels.
+of the three formats.  Only runnable with PCP_REFERENCE naming a reference checkout; the .npz
+travels.
 
-    python tests/golden/make_ply_fixtures.py
+    PCP_REFERENCE=<checkout> python tests/golden/make_ply_fixtures.py
 """
 import os
 import sys

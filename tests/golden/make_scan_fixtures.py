@@ -1,12 +1,12 @@
 """Generates tests/golden/ref_scans.npz: the reference's real scans
-(/root/reference/examples/data/{stanford_bunny,fandisk,detergent,spray}.ply, SURVEY.md §8c) read
+($PCP_REFERENCE/examples/data/{stanford_bunny,fandisk,detergent,spray}.ply, SURVEY.md §8c) read
 by the UNMODIFIED reference PLY reader and pushed through the UNMODIFIED reference octree and
 kd-tree (oracle/_ref/libpcp_ref*.so): full-cloud kNN k = 15 (indices + squared distances),
 sphere-range counts at r = 2 x the mean 15-NN distance, per-point mean 15-NN distance.  The
-clouds themselves are stored too (the scans do not travel to the GPU box).  Only runnable where
-/root/reference exists.
+clouds themselves are stored too (the scans are not part of this repository).  Only runnable
+with PCP_REFERENCE naming a reference checkout.
 
-    python tests/golden/make_scan_fixtures.py
+    PCP_REFERENCE=<checkout> python tests/golden/make_scan_fixtures.py
 """
 import os
 import sys
@@ -16,9 +16,9 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
 
-from oracle_lib import RefBridge, RefPly  # noqa: E402
+from oracle_lib import REFERENCE_DIR, RefBridge, RefPly  # noqa: E402
 
-DATA = "/root/reference/examples/data"
+DATA = os.path.join(REFERENCE_DIR or "$PCP_REFERENCE", "examples", "data")
 SCANS = ["stanford_bunny", "fandisk", "detergent", "spray"]
 
 

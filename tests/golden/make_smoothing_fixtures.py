@@ -1,9 +1,10 @@
 """Generates tests/golden/ref_smoothing.npz by running the UNMODIFIED reference
 (oracle/_ref/libpcp_ref_smoothing.so: pcp::algorithm::bilateral_filter_points and the
-pcp::algorithm::wlop::detail bodies, compiled in place from /root/reference/include) on small
-seeded clouds.  Only runnable where /root/reference exists; the committed .npz travels.
+pcp::algorithm::wlop::detail bodies, compiled in place from $PCP_REFERENCE/include) on small
+seeded clouds.  Only runnable with PCP_REFERENCE naming a reference checkout; the committed
+.npz travels.
 
-    python tests/golden/make_smoothing_fixtures.py
+    PCP_REFERENCE=<checkout> python tests/golden/make_smoothing_fixtures.py
 """
 import os
 import sys

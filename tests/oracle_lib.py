@@ -2,8 +2,8 @@
 
 * ``Oracle``   — oracle/liboracle.so, the plain-C restatement (oracle/pcp_oracle.c).
 * ``RefBridge`` — oracle/_ref/libpcp_ref.so, the UNMODIFIED reference headers behind a flat C
-  bridge (oracle/ref_bridge.cpp). Only buildable where /root/reference exists; the prebuilt
-  library travels to the GPU box with the snapshot.
+  bridge (oracle/ref_bridge.cpp). Only buildable when the environment variable PCP_REFERENCE
+  names a checkout of the reference (REFERENCE_DIR); a prebuilt oracle/_ref is used as it is.
 """
 import ctypes as C
 import os
@@ -18,6 +18,7 @@ REF_SO = os.path.join(ORACLE_DIR, "_ref", "libpcp_ref.so")
 REF_SMOOTHING_SO = os.path.join(ORACLE_DIR, "_ref", "libpcp_ref_smoothing.so")
 REF_ORIENT_SO = os.path.join(ORACLE_DIR, "_ref", "libpcp_ref_orient.so")
 REF_PLY_SO = os.path.join(ORACLE_DIR, "_ref", "libpcp_ref_ply.so")
+REFERENCE_DIR = os.environ.get("PCP_REFERENCE") or None  # a checkout of Q-Minh/point-cloud-processing
 
 _f32p = C.POINTER(C.c_float)
 _i64p = C.POINTER(C.c_int64)
@@ -38,7 +39,8 @@ def build_oracle(force=False):
     """Compile the checker libraries (make -C oracle). Building the checker is not using it."""
     src = os.path.join(ORACLE_DIR, "pcp_oracle.c")
     stale = (not os.path.exists(ORACLE_SO)) or os.path.getmtime(ORACLE_SO) < os.path.getmtime(src)
-    ref_possible = os.path.isdir("/root/reference/include/pcp")
+    ref_possible = REFERENCE_DIR is not None and os.path.isdir(
+        os.path.join(REFERENCE_DIR, "include", "pcp"))
     ref_src = os.path.join(ORACLE_DIR, "ref_bridge.cpp")
     ref_stale = ref_possible and (
         (not os.path.exists(REF_SO)) or os.path.getmtime(REF_SO) < os.path.getmtime(ref_src)

@@ -52,7 +52,8 @@ def test_oracle_matches_live_reference(oracle):
     from oracle_lib import RefOrient, have_ref_orient
 
     if not have_ref_orient():
-        pytest.skip("oracle/_ref/libpcp_ref_orient.so not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/libpcp_ref_orient.so not built (set PCP_REFERENCE to a reference "
+                    "checkout)")
     ref = RefOrient()
     rng = np.random.default_rng(6)
     xyz = np.stack([rng.uniform(0, 1, 3000), rng.uniform(0, 1, 3000),

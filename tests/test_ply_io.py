@@ -1,8 +1,8 @@
 """include/pcpx/ply.hpp (host-only PLY reader / writer, SURVEY.md §8f rank 4) against the
 reference's on-disk format: byte streams written by the UNMODIFIED reference writer
 (tests/golden/ref_ply.npz, made by make_ply_fixtures.py) must be read back exactly, and the
-writer must produce those same bytes.  Also the reference's real scans when /root/reference is
-mounted (CPU container only)."""
+writer must produce those same bytes.  Also the reference's real scans when PCP_REFERENCE
+names a checkout of the reference."""
 import os
 import struct
 import subprocess
@@ -103,12 +103,13 @@ def test_comments_doubles_and_extra_elements(tool, tmp_path):
 
 
 def test_reference_scans_when_mounted(tool, tmp_path):
-    data = "/root/reference/examples/data"
-    if not os.path.isdir(data):
-        pytest.skip("reference scans are only present in the CPU container")
+    from oracle_lib import REFERENCE_DIR, RefPly, have_ref_ply
+
+    data = os.path.join(REFERENCE_DIR, "examples", "data") if REFERENCE_DIR else None
+    if data is None or not os.path.isdir(data):
+        pytest.skip("the reference's example scans need PCP_REFERENCE (a reference checkout)")
     expected = {"stanford_bunny.ply": 35947, "detergent.ply": 20266, "spray.ply": 14851,
                 "fandisk.ply": 6475}
-    from oracle_lib import RefPly, have_ref_ply
 
     ref = RefPly() if have_ref_ply() else None
     for name, n in expected.items():

@@ -68,7 +68,8 @@ def test_oracle_matches_live_reference(oracle):
     from oracle_lib import RefSmoothing, have_ref_smoothing
 
     if not have_ref_smoothing():
-        pytest.skip("oracle/_ref/libpcp_ref_smoothing.so not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/libpcp_ref_smoothing.so not built (set PCP_REFERENCE to a reference "
+                    "checkout)")
     ref = RefSmoothing()
     rng = np.random.default_rng(77)
     xyz = np.stack([rng.uniform(0, 1, 2500), rng.uniform(0, 1, 2500),
