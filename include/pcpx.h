@@ -241,6 +241,52 @@ int pcpx_estimate_tangent_planes(
     float* out_normals);
 
 /*
+ * Fused ball -> 3x3 scatter matrix -> symmetric eigensolve -> normal, in one device pass with
+ * no per-neighbour data in memory.  Replaces pcp::algorithm::estimate_normals
+ * (algorithm/estimate_normals.hpp:50-93,116-164) driven by a sphere range-search map,
+ * `[&](auto const& p) { return octree.range_search(sphere_t{p, r}, point_view); }`
+ * (octree/linked_octree.hpp:264-276, predicate common/sphere.hpp:27-35), with
+ * pcp::estimate_normal (common/normals/normal_estimation.hpp:32-78) as the per-ball body.
+ *   - the ball of query i is exactly the set pcpx_radius_search returns for it: the indexed
+ *     points with fl(d2) <= fl(r*r), the query itself included when it is an indexed point;
+ *     points a voxel grid left out of the index are in no ball but are valid queries.
+ *   - radii != NULL gives one radius per query, else `radius` is used.
+ *   - per ball: fp32 mean, centred UN-normalised scatter, unit eigenvector of the smallest
+ *     eigenvalue.  The sign is not canonical: compare with |dot|.  A ball of 0 or 1 points (zero
+ *     scatter) gives (0,0,1).
+ *   - out_count (nq entries, may be NULL) = the ball's size, equal to pcpx_radius_count.
+ * Note: the reference prunes with d2 <= r (common/intersections.hpp:101) and can therefore
+ * MISS in-range points when r > 1; this library always uses the exact ball.
+ * out_normals: nq x 3 fp32.  Runs on the primary device of a multi-device index.
+ */
+int pcpx_estimate_normals_radius(
+    const pcpx_index* index,
+    const float* queries,
+    size_t nq,
+    size_t query_stride_bytes,
+    const float* radii,
+    float radius,
+    float* out_normals,
+    uint32_t* out_count);
+
+/*
+ * As pcpx_estimate_normals_radius, and also writes the ball's centroid: the tangent plane
+ * (point, normal) of pcp::algorithm::estimate_tangent_planes
+ * (algorithm/estimate_tangent_planes.hpp:82-94) with a sphere range-search map.  An empty ball
+ * gives a NaN centroid, normal (0,0,1) and count 0.  out_points: nq x 3 fp32.
+ */
+int pcpx_estimate_tangent_planes_radius(
+    const pcpx_index* index,
+    const float* queries,
+    size_t nq,
+    size_t query_stride_bytes,
+    const float* radii,
+    float radius,
+    float* out_points,
+    float* out_normals,
+    uint32_t* out_count);
+
+/*
  * PCA normal of caller-supplied neighbourhoods (CSR: neighbourhood i = points
  * nbr_xyz[offsets[i] .. offsets[i + 1]), packed fp32 xyz).  This is pcp::estimate_normal
  * (common/normals/normal_estimation.hpp:32-78) batched on the GPU; it serves

@@ -13,7 +13,8 @@
 //   * every query has a BATCHED overload next to the per-query one; the per-query overloads
 //     cost one kernel launch each and exist for source compatibility,
 //   * `estimate_normals` recognises `pcp::gpu_knn_map` (an index + k) and then runs the fused
-//     kNN -> PCA kernel once for the whole range; with any other KnnMap it calls the map per
+//     kNN -> PCA kernel once for the whole range, and `pcp::gpu_radius_map` (an index + a
+//     radius) the fused ball -> PCA kernel; with any other KnnMap it calls the map per
 //     element like the reference does and batches only the PCA (still on the GPU),
 //   * failures throw std::runtime_error (the reference has no error path at all); there is no
 //     CPU fallback anywhere.
@@ -993,6 +994,45 @@ struct is_gpu_knn_map<gpu_knn_map<I, P>> : std::true_type
 };
 } // namespace detail
 
+// The ball counterpart: a KnnMap bound to a device index and a radius.  Called on one element it
+// answers like `[&](auto const& e) { return index.range_search(sphere_t{point_view(e), radius},
+// point_view); }` (octree/linked_octree.hpp:264-276, common/sphere.hpp:27-35); handed to
+// estimate_normals it makes the whole range one fused ball -> PCA device call.
+template <class Index, class PointViewMap>
+struct gpu_radius_map
+{
+    Index const* index;
+    float radius;
+    PointViewMap point_view;
+
+    template <class Key>
+    std::vector<typename Index::element_type> operator()(Key const& key) const
+    {
+        std::vector<float> c, r{radius};
+        detail::push_xyz(c, point_view(key));
+        std::vector<std::uint64_t> off;
+        std::vector<std::uint32_t> idx;
+        index->radius_batch(c, r, off, idx);
+        return index->gather(idx.data(), idx.size());
+    }
+};
+template <class Index, class PointViewMap>
+gpu_radius_map<Index, PointViewMap> make_gpu_radius_map(Index const& index, float radius,
+                                                        PointViewMap point_view)
+{
+    return gpu_radius_map<Index, PointViewMap>{&index, radius, point_view};
+}
+namespace detail {
+template <class T>
+struct is_gpu_radius_map : std::false_type
+{
+};
+template <class I, class P>
+struct is_gpu_radius_map<gpu_radius_map<I, P>> : std::true_type
+{
+};
+} // namespace detail
+
 // common/normals/normal_estimation.hpp:32-78 for ONE neighbourhood (a device call; batch instead)
 template <class ForwardIter, class PointViewMap, class Normal = pcp::normal_t>
 Normal estimate_normal(ForwardIter it, ForwardIter end, PointViewMap const& point_map)
@@ -1024,9 +1064,9 @@ void estimate_normals(ForwardIter1 begin, ForwardIter1 end, ForwardIter2 out_beg
     using knn_type      = std::decay_t<KnnMap>;
     std::size_t const n = static_cast<std::size_t>(std::distance(begin, end));
     detail::pinned_buffer<float> normals(3 * n);
-    if constexpr (detail::is_gpu_knn_map<knn_type>::value)
+    if constexpr (detail::is_gpu_knn_map<knn_type>::value || detail::is_gpu_radius_map<knn_type>::value)
     {
-        // the whole range in ONE fused kNN -> scatter matrix -> eigensolve call
+        // the whole range in ONE fused kNN (or ball) -> scatter matrix -> eigensolve call
         detail::pinned_buffer<float> q(3 * n);
         auto const put = [&](std::size_t i, auto const& element) {
             auto const p = point_map(element);
@@ -1047,10 +1087,16 @@ void estimate_normals(ForwardIter1 begin, ForwardIter1 end, ForwardIter2 out_beg
         // the range is the indexed cloud itself (the usual call): no query upload, no query
         // sort, the tile kernel
         bool const own = knn_map.index->is_own_cloud(q.data(), n);
-        detail::check(pcpx_estimate_normals(knn_map.index->handle(), own ? nullptr : q.data(), n, 12,
-                                            static_cast<std::uint32_t>(knn_map.k), knn_map.eps,
-                                            normals.data()),
-                      "pcpx_estimate_normals");
+        if constexpr (detail::is_gpu_knn_map<knn_type>::value)
+            detail::check(pcpx_estimate_normals(knn_map.index->handle(), own ? nullptr : q.data(), n,
+                                                12, static_cast<std::uint32_t>(knn_map.k),
+                                                knn_map.eps, normals.data()),
+                          "pcpx_estimate_normals");
+        else
+            detail::check(pcpx_estimate_normals_radius(knn_map.index->handle(),
+                                                       own ? nullptr : q.data(), n, 12, nullptr,
+                                                       knn_map.radius, normals.data(), nullptr),
+                          "pcpx_estimate_normals_radius");
     }
     else
     {

@@ -83,6 +83,11 @@ _SIGNATURES = {
                                         C.c_uint32, C.c_double, C.c_void_p]),
     "pcpx_estimate_tangent_planes": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t,
                                                C.c_uint32, C.c_double, C.c_void_p, C.c_void_p]),
+    "pcpx_estimate_normals_radius": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t,
+                                               C.c_void_p, C.c_float, C.c_void_p, C.c_void_p]),
+    "pcpx_estimate_tangent_planes_radius": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t,
+                                                      C.c_size_t, C.c_void_p, C.c_float,
+                                                      C.c_void_p, C.c_void_p, C.c_void_p]),
     "pcpx_normals_from_neighbourhoods": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int,
                                                    C.c_void_p]),
     "pcpx_mean_knn_distance": (C.c_int, [C.c_void_p, C.c_uint32, C.c_double, C.c_void_p,
@@ -422,6 +427,36 @@ class Index:
         _check(lib().pcpx_estimate_tangent_planes(self._h, q.ptr, nq, 12, k, eps,
                                                   pts.ctypes.data, nrm.ctypes.data))
         return pts, nrm
+
+    def estimate_normals_radius(self, queries, radius, radii=None, out=None, out_count=None):
+        """PCA normal of every query's ball (the set radius_search returns); `radii` gives one
+        radius per query.  Results are numpy arrays, or CUDA tensors when the queries are;
+        out_count, when given, receives the ball sizes."""
+        nq = self._nq(queries)
+        q = _Buf(queries, np.float32)
+        r = _Buf(radii, np.float32)
+        out = _out_rows(queries, nq, out)
+        bo, bc = _Buf(out, np.float32, True), _Buf(out_count, np.uint32, True)
+        _check(lib().pcpx_estimate_normals_radius(self._h, q.ptr, nq, 12, r.ptr, float(radius),
+                                                  bo.ptr, bc.ptr))
+        return out
+
+    def estimate_tangent_planes_radius(self, queries, radius, radii=None):
+        """(centroids, normals, counts) of every query's ball; an empty ball gives a NaN
+        centroid, normal (0,0,1) and count 0."""
+        nq = self._nq(queries)
+        q = _Buf(queries, np.float32)
+        r = _Buf(radii, np.float32)
+        pts, nrm = _out_rows(queries, nq, None), _out_rows(queries, nq, None)
+        if _is_torch(queries):
+            import torch
+            cnt = torch.empty(nq, dtype=torch.int32, device=queries.device)
+        else:
+            cnt = np.zeros(nq, np.uint32)
+        bp, bn, bc = _Buf(pts, np.float32, True), _Buf(nrm, np.float32, True), _Buf(cnt)
+        _check(lib().pcpx_estimate_tangent_planes_radius(self._h, q.ptr, nq, 12, r.ptr,
+                                                         float(radius), bp.ptr, bn.ptr, bc.ptr))
+        return pts, nrm, cnt
 
     def mean_knn_distance(self, k, eps=1e-5):
         per = np.zeros(self.n, np.float32)

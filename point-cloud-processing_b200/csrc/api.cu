@@ -549,6 +549,58 @@ int pcpx_estimate_tangent_planes(const pcpx_index* index, const float* queries, 
     });
 }
 
+static void radius_normals_impl(const pcpx_index* index, const float* queries, size_t nq,
+                                size_t query_stride_bytes, const float* radii, float radius,
+                                float* out_points, float* out_normals, uint32_t* out_count)
+{
+    pcpx_index& ix = checked(index);
+    if (nq == 0)
+        return;
+    if (!out_normals)
+        fail(PCPX_ERR_INVALID_ARG, "out_normals is NULL");
+    ScopedDevice guard(ix.device);
+    CallStream call(ix); // own stream: calls on one index may run concurrently
+    CallTimer timer(ix);
+    Batch batch;
+    batch.prepare(ix, queries, nq, query_stride_bytes);
+    InBuf rad;
+    rad.stage(radii, nq, 4, 1, ix.qstream());
+    OutBuf<float> nrm, ctr;
+    OutBuf<uint32_t> cnt;
+    nrm.prepare(out_normals, nq * 3);
+    ctr.prepare(out_points, nq * 3);
+    cnt.prepare(out_count, nq);
+    timer.kernel_begin();
+    launch_radius_normals(ix, batch.qb, rad.d, radius, nrm.d, ctr.d, cnt.d);
+    timer.kernel_end();
+    ix.timings.kernel_launches = 1;
+    nrm.finish(ix.qstream()), ctr.finish(ix.qstream()), cnt.finish(ix.qstream());
+    timer.done();
+}
+
+int pcpx_estimate_normals_radius(const pcpx_index* index, const float* queries, size_t nq,
+                                 size_t query_stride_bytes, const float* radii, float radius,
+                                 float* out_normals, uint32_t* out_count)
+{
+    return guarded([&] {
+        radius_normals_impl(index, queries, nq, query_stride_bytes, radii, radius, nullptr,
+                            out_normals, out_count);
+    });
+}
+
+int pcpx_estimate_tangent_planes_radius(const pcpx_index* index, const float* queries, size_t nq,
+                                        size_t query_stride_bytes, const float* radii,
+                                        float radius, float* out_points, float* out_normals,
+                                        uint32_t* out_count)
+{
+    return guarded([&] {
+        if (nq && !out_points)
+            fail(PCPX_ERR_INVALID_ARG, "out_points is NULL");
+        radius_normals_impl(index, queries, nq, query_stride_bytes, radii, radius, out_points,
+                            out_normals, out_count);
+    });
+}
+
 int pcpx_normals_from_neighbourhoods(const float* nbr_xyz, const uint64_t* offsets, size_t n,
                                      int device, float* out_normals)
 {

@@ -1,8 +1,9 @@
 // Per-query epilogues on top of the top-K list: PCA normal / tangent plane and mean neighbour
-// distance.  __host__ __device__ (see grid_core.cuh).
+// distance; the PCA over a radius ball.  __host__ __device__ (see grid_core.cuh).
 #pragma once
 #include "eig3.cuh"
 #include "knn_core.cuh"
+#include "radius_core.cuh"
 
 namespace pcpx {
 
@@ -112,6 +113,40 @@ PCPX_HD bool normal_two_pass(const GridView& g, const Region& region, const SL& 
     if (centroid3)
         centroid3[0] = qx + mx, centroid3[1] = qy + my, centroid3[2] = qz + mz;
     return true;
+}
+
+// The same PCA over a ball: exactly the points pcpx_radius_search returns for (q, r), the query
+// itself included when it is an indexed point (radius_visit).  One walk accumulates the moments
+// about the query point as above (the ball surrounds the query), so no per-neighbour data is
+// kept anywhere.  n == 0: NaN centroid and (0,0,1); n == 1: the reference's centred scatter of a
+// single point is exactly zero -> (0,0,1) (the shifted form would leave rounding residue).
+// Returns n.
+PCPX_HD uint32_t radius_normal(const GridView& g, float qx, float qy, float qz, float r, float* n3,
+                               float* centroid3)
+{
+    uint32_t n = 0;
+    float s1x = 0.f, s1y = 0.f, s1z = 0.f;
+    Sym3 s2{0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    radius_visit(g, qx, qy, qz, r, [&](float4 const& c, uint32_t) {
+        float const dx = c.x - qx, dy = c.y - qy, dz = c.z - qz;
+        ++n;
+        s1x += dx, s1y += dy, s1z += dz;
+        s2.xx += dx * dx, s2.xy += dx * dy, s2.xz += dx * dz;
+        s2.yy += dy * dy, s2.yz += dy * dz, s2.zz += dz * dz;
+        return false;
+    });
+    float const inv = 1.f / (float)n; // n == 0: NaN centroid
+    float const mx = s1x * inv, my = s1y * inv, mz = s1z * inv;
+    Sym3 m{0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    if (n > 1)
+    {
+        m.xx = s2.xx - s1x * mx, m.xy = s2.xy - s1x * my, m.xz = s2.xz - s1x * mz;
+        m.yy = s2.yy - s1y * my, m.yz = s2.yz - s1y * mz, m.zz = s2.zz - s1z * mz;
+    }
+    smallest_eigenvector_fast(m, n3[0], n3[1], n3[2]);
+    if (centroid3)
+        centroid3[0] = qx + mx, centroid3[1] = qy + my, centroid3[2] = qz + mz;
+    return n;
 }
 
 // Second pass of the kNN kernel: every neighbour goes straight to its rank in the output row.

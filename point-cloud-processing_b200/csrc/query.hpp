@@ -60,6 +60,10 @@ void launch_mean_distance(const pcpx_index& ix, const QueryBatch& qb, uint32_t k
                           float* means);
 void launch_radius_count(const pcpx_index& ix, const QueryBatch& qb, const float* radii, float r,
                          uint32_t* count);
+// PCA normal of every query's ball (normals: nq x 3; centroids: nq x 3 or nullptr; count: nq or
+// nullptr), rows as launch_radius_count
+void launch_radius_normals(const pcpx_index& ix, const QueryBatch& qb, const float* radii, float r,
+                           float* normals, float* centroids, uint32_t* count);
 void launch_radius_fill(const pcpx_index& ix, const QueryBatch& qb, const float* radii, float r,
                         const uint64_t* offsets, uint32_t* idx);
 // dst[row(t) * width + j] = src[t * width + j] for the sorted positions t a shard answered (see
