@@ -204,6 +204,41 @@ int pcpx_radius_search(
     uint32_t** out_idx,
     int out_idx_device);
 
+/*
+ * Axis-aligned box range search.  Replaces range_search(axis_aligned_bounding_box_t)
+ * (octree/linked_octree.hpp:264-276 -> octree/linked_octree_node.hpp:581-614) and
+ * range_search(kd_axis_aligned_bounding_box_t) (kdtree/linked_kdtree.hpp:270-316), with predicate
+ * axis_aligned_bounding_box_t::contains (common/axis_aligned_bounding_box.hpp:99-149).
+ *   - boxes: nb records of 6 fp32 {min x, min y, min z, max x, max y, max z}, box_stride_bytes
+ *     (>= 24, a multiple of 4) apart, in host or device memory.
+ *   - box b's result: the indexed points p with min <= p <= max on all three axes, compared in
+ *     fp32 (inclusive on both ends); points a voxel grid left out of the index are in no box.
+ *   - a box with a NaN bound or min > max on some axis is empty; +-inf bounds are valid.
+ * pcpx_box_count: out_count (nb entries) = the size of every box's result.
+ */
+int pcpx_box_count(
+    const pcpx_index* index,
+    const float* boxes,
+    size_t nb,
+    size_t box_stride_bytes,
+    uint32_t* out_count);
+
+/*
+ * Box range search, CSR lists (out_offsets: nb + 1 entries), flags as pcpx_radius_search:
+ * PCPX_RADIUS_DEVICE leaves *out_idx in device memory, PCPX_RADIUS_SORTED sorts every list
+ * ascending by original index; without it a list is in the index's traversal order
+ * (deterministic, unspecified).  Free *out_idx with pcpx_free.  Runs on the primary device of a
+ * multi-device index.
+ */
+int pcpx_box_search(
+    const pcpx_index* index,
+    const float* boxes,
+    size_t nb,
+    size_t box_stride_bytes,
+    uint64_t* out_offsets,
+    uint32_t** out_idx,
+    int flags);
+
 void pcpx_free(void* p, int is_device);
 
 /*

@@ -516,6 +516,36 @@ inline index_ptr make_index(float const* xyz, std::size_t n, pcpx_index_params c
     check(pcpx_index_create(xyz, n, 12, &prm, &raw), "pcpx_index_create");
     return index_ptr(raw);
 }
+// fp32 bounds that contain [v, v] when v is wider than float
+template <class T>
+float round_down_f32(T v)
+{
+    float const f = static_cast<float>(v);
+    if constexpr (std::is_same_v<T, float>)
+        return f;
+    else
+        return static_cast<T>(f) > v ? std::nextafter(f, -std::numeric_limits<float>::infinity()) : f;
+}
+template <class T>
+float round_up_f32(T v)
+{
+    float const f = static_cast<float>(v);
+    if constexpr (std::is_same_v<T, float>)
+        return f;
+    else
+        return static_cast<T>(f) < v ? std::nextafter(f, std::numeric_limits<float>::infinity()) : f;
+}
+template <class R, class = void>
+struct is_aabb : std::false_type
+{
+};
+template <class R>
+struct is_aabb<R, std::void_t<decltype(std::declval<R const&>().min),
+                              decltype(std::declval<R const&>().max)>> : std::true_type
+{
+};
+template <class R>
+inline constexpr bool is_aabb_v = is_aabb<R>::value;
 template <class PV>
 void push_xyz(std::vector<float>& out, PV const& p)
 {
@@ -607,6 +637,30 @@ class device_spatial_index
                       "pcpx_radius_search");
         idx.assign(lists, lists + offsets[n]);
         pcpx_free(lists, 0);
+    }
+
+    // box range search, CSR over original indices, every list ascending
+    void box_batch(std::vector<float> const& boxes, std::vector<std::uint64_t>& offsets,
+                   std::vector<std::uint32_t>& idx) const
+    {
+        std::size_t const n = boxes.size() / 6;
+        offsets.assign(n + 1, 0u);
+        std::uint32_t* lists = nullptr;
+        detail::check(pcpx_box_search(index_.get(), boxes.data(), n, 24, offsets.data(), &lists,
+                                      PCPX_RADIUS_SORTED),
+                      "pcpx_box_search");
+        idx.assign(lists, lists + offsets[n]);
+        pcpx_free(lists, 0);
+    }
+    // one box as 6 fp32 values, rounded outward when the coordinates are wider than float (a
+    // NaN bound stays NaN: the box is empty either way)
+    template <class T>
+    static void push_box(std::vector<float>& out, T const (&mn)[3], T const (&mx)[3])
+    {
+        for (int a = 0; a < 3; ++a)
+            out.push_back(detail::round_down_f32(mn[a]));
+        for (int a = 0; a < 3; ++a)
+            out.push_back(detail::round_up_f32(mx[a]));
     }
 
   protected:
@@ -785,46 +839,54 @@ class basic_linked_octree_t : public device_spatial_index<Element>
         return this->gather(idx.data(), idx.size());
     }
 
-    // ... and for the box range: GPU search of the circumscribed sphere, exact box predicate after
+    // ... and for the box range (pcpx_box_search)
     template <class Point, class PointViewMap>
     std::vector<element_type> range_search(axis_aligned_bounding_box_t<Point> const& range,
                                            PointViewMap const& point_view) const
     {
-        float const hx = 0.5f * (range.max.x() - range.min.x()),
-                    hy = 0.5f * (range.max.y() - range.min.y()),
-                    hz = 0.5f * (range.max.z() - range.min.z());
-        std::vector<float> c{range.min.x() + hx, range.min.y() + hy, range.min.z() + hz};
-        // the centre is rounded to fp32 (up to half an ulp of its magnitude per axis) and the
-        // device evaluates fp32 distances: absolute slack of a few ulps of the largest
-        // coordinate on top of the relative margin, so that a small box far from the origin
-        // still sees the points in its corners
-        float const big = std::max({std::fabs(range.min.x()), std::fabs(range.max.x()),
-                                    std::fabs(range.min.y()), std::fabs(range.max.y()),
-                                    std::fabs(range.min.z()), std::fabs(range.max.z())});
-        std::vector<float> r{std::sqrt(hx * hx + hy * hy + hz * hz) * 1.0001f + 8.f * 1.1920929e-7f * big +
-                             1e-30f};
+        std::vector<float> b;
+        this->push_box(b, {range.min.x(), range.min.y(), range.min.z()},
+                       {range.max.x(), range.max.y(), range.max.z()});
         std::vector<std::uint64_t> off;
         std::vector<std::uint32_t> idx;
-        this->radius_batch(c, r, off, idx);
-        std::vector<element_type> out;
-        for (auto i : idx)
-            if (range.contains(point_view(this->elements_[i])))
-                out.push_back(this->elements_[i]);
-        return out;
+        this->box_batch(b, off, idx);
+        if constexpr (std::is_same_v<std::decay_t<decltype(range.min.x())>, float>)
+            return this->gather(idx.data(), idx.size());
+        else
+        {
+            // the box was rounded outward to fp32: the exact predicate on what it returned
+            std::vector<element_type> out;
+            for (auto i : idx)
+                if (range.contains(point_view(this->elements_[i])))
+                    out.push_back(this->elements_[i]);
+            return out;
+        }
     }
 
-    // batched sphere ranges -> CSR (offsets, original indices)
-    template <class SphereIter>
-    void range_search(SphereIter begin, SphereIter end, std::vector<std::uint64_t>& offsets,
+    // batched sphere or box ranges -> CSR (offsets, original indices), every list ascending
+    template <class RangeIter>
+    void range_search(RangeIter begin, RangeIter end, std::vector<std::uint64_t>& offsets,
                       std::vector<std::uint32_t>& indices) const
     {
-        std::vector<float> c, r;
-        for (auto it = begin; it != end; ++it)
+        using range_type = typename std::iterator_traits<RangeIter>::value_type;
+        if constexpr (detail::is_aabb_v<range_type>)
         {
-            detail::push_xyz(c, it->position);
-            r.push_back(static_cast<float>(it->radius));
+            std::vector<float> b;
+            for (auto it = begin; it != end; ++it)
+                this->push_box(b, {it->min.x(), it->min.y(), it->min.z()},
+                               {it->max.x(), it->max.y(), it->max.z()});
+            this->box_batch(b, offsets, indices);
         }
-        this->radius_batch(c, r, offsets, indices);
+        else
+        {
+            std::vector<float> c, r;
+            for (auto it = begin; it != end; ++it)
+            {
+                detail::push_xyz(c, it->position);
+                r.push_back(static_cast<float>(it->radius));
+            }
+            this->radius_batch(c, r, offsets, indices);
+        }
     }
 
   private:
@@ -913,31 +975,53 @@ class basic_linked_kdtree_t : public device_spatial_index<Element>
         }
         return this->knn_batch(q, k, static_cast<double>(eps));
     }
-    // ... and for the kd box range: circumscribed sphere on the GPU, exact box predicate after
+    // kdtree/linked_kdtree.hpp:270-316 for the kd box range (pcpx_box_search).  Coordinates other
+    // than float: the box is rounded outward to fp32 and the exact predicate filters the result.
     std::vector<element_type>
     range_search(kd_axis_aligned_bounding_box_t<coordinate_type, 3> const& range) const
     {
-        float h[3], c[3];
-        for (int a = 0; a < 3; ++a)
-        {
-            h[a] = 0.5f * static_cast<float>(range.max[a] - range.min[a]);
-            c[a] = static_cast<float>(range.min[a]) + h[a];
-        }
-        std::vector<float> cc{c[0], c[1], c[2]};
-        float big = 0.f; // see the octree's box overload: slack for the rounded centre
-        for (int a = 0; a < 3; ++a)
-            big = std::max({big, std::fabs(static_cast<float>(range.min[a])),
-                            std::fabs(static_cast<float>(range.max[a]))});
-        std::vector<float> r{std::sqrt(h[0] * h[0] + h[1] * h[1] + h[2] * h[2]) * 1.0001f +
-                             8.f * 1.1920929e-7f * big + 1e-30f};
+        std::vector<float> b;
+        this->push_box(b, {range.min[0], range.min[1], range.min[2]},
+                       {range.max[0], range.max[1], range.max[2]});
         std::vector<std::uint64_t> off;
         std::vector<std::uint32_t> idx;
-        this->radius_batch(cc, r, off, idx);
-        std::vector<element_type> out;
-        for (auto i : idx)
-            if (range.contains(coordinate_map_(this->elements_[i])))
-                out.push_back(this->elements_[i]);
-        return out;
+        this->box_batch(b, off, idx);
+        if constexpr (std::is_same_v<coordinate_type, float>)
+            return this->gather(idx.data(), idx.size());
+        else
+        {
+            std::vector<element_type> out;
+            for (auto i : idx)
+                if (range.contains(coordinate_map_(this->elements_[i])))
+                    out.push_back(this->elements_[i]);
+            return out;
+        }
+    }
+    // batched kd boxes -> CSR (offsets, original indices), every list ascending; non-float
+    // coordinates as above, with each list filtered by the exact predicate
+    template <class BoxIter>
+    void range_search(BoxIter begin, BoxIter end, std::vector<std::uint64_t>& offsets,
+                      std::vector<std::uint32_t>& indices) const
+    {
+        std::vector<float> b;
+        for (auto it = begin; it != end; ++it)
+            this->push_box(b, {it->min[0], it->min[1], it->min[2]},
+                           {it->max[0], it->max[1], it->max[2]});
+        this->box_batch(b, offsets, indices);
+        if constexpr (!std::is_same_v<coordinate_type, float>)
+        {
+            std::vector<std::uint64_t> off{0u};
+            std::vector<std::uint32_t> kept;
+            std::size_t q = 0;
+            for (auto it = begin; it != end; ++it, ++q)
+            {
+                for (std::uint64_t j = offsets[q]; j < offsets[q + 1]; ++j)
+                    if (it->contains(coordinate_map_(this->elements_[indices[j]])))
+                        kept.push_back(indices[j]);
+                off.push_back(kept.size());
+            }
+            offsets.swap(off), indices.swap(kept);
+        }
     }
     // kdtree/linked_kdtree.hpp:270-277 for sphere_a
     std::vector<element_type> range_search(sphere_a<coordinate_type> const& range) const

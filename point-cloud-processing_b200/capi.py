@@ -78,6 +78,9 @@ _SIGNATURES = {
                                     C.c_float, C.c_void_p]),
     "pcpx_radius_search": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p,
                                      C.c_float, C.c_void_p, C.POINTER(C.c_void_p), C.c_int]),
+    "pcpx_box_count": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p]),
+    "pcpx_box_search": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p,
+                                  C.POINTER(C.c_void_p), C.c_int]),
     "pcpx_free": (None, [C.c_void_p, C.c_int]),
     "pcpx_estimate_normals": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t,
                                         C.c_uint32, C.c_double, C.c_void_p]),
@@ -288,6 +291,12 @@ def _count(x):
     return x.shape[0] if x.ndim == 2 else x.size // 3
 
 
+def _count_boxes(x):
+    if _is_torch(x):
+        return x.numel() // 6
+    return np.asarray(x).size // 6
+
+
 class Index:
     """GPU-resident spatial index over a cloud (include/pcpx.h: pcpx_index_create)."""
 
@@ -402,6 +411,38 @@ class Index:
         p = C.c_void_p()
         _check(lib().pcpx_radius_search(self._h, q.ptr, nq, 12, r.ptr, float(radius),
                                         off.ctypes.data, C.byref(p), 2 if sorted else 0))
+        total = int(off[-1])
+        try:
+            idx = np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_uint32)),
+                                        shape=(max(total, 1),))[:total].copy()
+        finally:
+            lib().pcpx_free(p, 0)
+        return off, idx
+
+    def box_count(self, boxes, out_count=None):
+        """Size of every box's result; `boxes` is (nb, 6) {min xyz, max xyz}, a numpy array or a
+        CUDA tensor (then the counts are a CUDA tensor too, unless out_count is given)."""
+        nb = _count_boxes(boxes)
+        b = _Buf(boxes, np.float32)
+        if out_count is None:
+            if _is_torch(boxes):
+                import torch
+                out_count = torch.empty(nb, dtype=torch.int32, device=boxes.device)
+            else:
+                out_count = np.zeros(nb, np.uint32)
+        bc = _Buf(out_count, np.uint32, True)
+        _check(lib().pcpx_box_count(self._h, b.ptr, nb, 24, bc.ptr))
+        return out_count
+
+    def box_search(self, boxes, sorted=False):
+        """CSR (offsets[nb + 1], indices) of the indexed points inside every box — host arrays;
+        sorted: every list ascending by index (PCPX_RADIUS_SORTED), otherwise traversal order."""
+        nb = _count_boxes(boxes)
+        b = _Buf(boxes, np.float32)
+        off = np.zeros(nb + 1, np.uint64)
+        p = C.c_void_p()
+        _check(lib().pcpx_box_search(self._h, b.ptr, nb, 24, off.ctypes.data, C.byref(p),
+                                     2 if sorted else 0))
         total = int(off[-1])
         try:
             idx = np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_uint32)),

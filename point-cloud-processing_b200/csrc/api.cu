@@ -467,6 +467,116 @@ int pcpx_radius_search(const pcpx_index* index, const float* queries, size_t nq,
     });
 }
 
+// the boxes of a box call, staged; bb = the index's bounding box (its voxel grid when it has one),
+// which holds every indexed point
+static BoxBatch box_batch(pcpx_index& ix, const float* boxes, size_t nb, size_t stride_bytes,
+                          InBuf& in)
+{
+    if (nb >= 0xFFFFFFFFull)
+        fail(PCPX_ERR_UNSUPPORTED, "more than 2^32 - 2 boxes in one call");
+    if (nb && !boxes)
+        fail(PCPX_ERR_INVALID_ARG, "boxes is NULL");
+    in.stage(boxes, nb, stride_bytes, 6, ix.qstream());
+    BoxBatch bx{in.d, in.stride_f, (uint32_t)nb, {}};
+    for (int a = 0; a < 3; ++a)
+        bx.bb[a] = ix.bbox_min[a], bx.bb[3 + a] = ix.bbox_max[a];
+    return bx;
+}
+
+static void check_box_stride(size_t stride_bytes)
+{
+    if (stride_bytes < 24 || stride_bytes % 4)
+        fail(PCPX_ERR_INVALID_ARG, "box_stride_bytes must be a multiple of 4 and >= 24");
+}
+
+int pcpx_box_count(const pcpx_index* index, const float* boxes, size_t nb,
+                   size_t box_stride_bytes, uint32_t* out_count)
+{
+    return guarded([&] {
+        pcpx_index& ix = checked(index);
+        if (!out_count)
+            fail(PCPX_ERR_INVALID_ARG, "out_count is NULL");
+        check_box_stride(box_stride_bytes);
+        if (nb == 0)
+            return;
+        ScopedDevice guard(ix.device);
+        CallStream call(ix); // own stream: calls on one index may run concurrently
+        CallTimer timer(ix);
+        InBuf in;
+        BoxBatch const bx = box_batch(ix, boxes, nb, box_stride_bytes, in);
+        OutBuf<uint32_t> cnt;
+        cnt.prepare(out_count, nb);
+        timer.kernel_begin();
+        launch_box_count(ix, bx, cnt.d, nullptr);
+        timer.kernel_end();
+        ix.timings.kernel_launches = 1;
+        cnt.finish(ix.qstream());
+        timer.done();
+    });
+}
+
+int pcpx_box_search(const pcpx_index* index, const float* boxes, size_t nb,
+                    size_t box_stride_bytes, uint64_t* out_offsets, uint32_t** out_idx, int flags)
+{
+    return guarded([&] {
+        pcpx_index& ix = checked(index);
+        if (!out_offsets || !out_idx)
+            fail(PCPX_ERR_INVALID_ARG, "out_offsets / out_idx is NULL");
+        *out_idx = nullptr;
+        check_box_stride(box_stride_bytes);
+        ScopedDevice guard(ix.device);
+        CallStream call(ix); // own stream: calls on one index may run concurrently
+        CallTimer timer(ix);
+        InBuf in;
+        BoxBatch const bx = box_batch(ix, boxes, nb, box_stride_bytes, in);
+        DevBuf<uint32_t> cnt(std::max<size_t>(nb, 1));
+        DevBuf<uint32_t> max_cnt(1);
+        PCPX_CUDA(cudaMemsetAsync(max_cnt.get(), 0, 4, ix.qstream()));
+        OutBuf<uint64_t> off;
+        off.prepare(out_offsets, nb + 1);
+        timer.kernel_begin();
+        launch_box_count(ix, bx, cnt.get(), max_cnt.get());
+        launch_exclusive_scan_u32(ix, cnt.get(), (uint32_t)nb, off.d);
+        uint64_t total = 0;
+        uint32_t longest = 0;
+        PCPX_CUDA(cudaMemcpyAsync(&total, off.d + nb, 8, cudaMemcpyDeviceToHost, ix.qstream()));
+        PCPX_CUDA(cudaMemcpyAsync(&longest, max_cnt.get(), 4, cudaMemcpyDeviceToHost, ix.qstream()));
+        PCPX_CUDA(cudaStreamSynchronize(ix.qstream()));
+        DevBuf<uint32_t> lists(std::max<uint64_t>(total, 1));
+        // count + the scan's three kernels + fill and copy + the sort's
+        uint32_t launches = nb ? 4 : 0;
+        launches += launch_box_fill(ix, bx, off.d, total, lists.get());
+        if (flags & PCPX_RADIUS_SORTED)
+            launches += launch_box_sort(ix, off.d, (uint32_t)nb, total, longest, lists.get());
+        timer.kernel_end();
+        ix.timings.kernel_launches = launches;
+        off.finish(ix.qstream());
+        if (flags & PCPX_RADIUS_DEVICE)
+        {
+            timer.done();
+            *out_idx = lists.detach();
+        }
+        else
+        {
+            uint32_t* host = (uint32_t*)std::malloc(std::max<uint64_t>(total, 1) * 4);
+            if (!host)
+                fail(PCPX_ERR_OUT_OF_MEMORY, "host allocation of %llu indices failed",
+                     (unsigned long long)total);
+            cudaError_t e = cudaMemcpyAsync(host, lists.get(), total * 4, cudaMemcpyDeviceToHost,
+                                            ix.qstream());
+            if (e == cudaSuccess)
+                e = cudaStreamSynchronize(ix.qstream());
+            if (e != cudaSuccess)
+            {
+                std::free(host);
+                fail(PCPX_ERR_CUDA, "copying box lists back failed: %s", cudaGetErrorString(e));
+            }
+            timer.done();
+            *out_idx = host;
+        }
+    });
+}
+
 void pcpx_free(void* p, int is_device)
 {
     if (!p)

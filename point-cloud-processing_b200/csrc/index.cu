@@ -564,4 +564,25 @@ void sort_queries_by_cell(const pcpx_index& ix, const float* d_queries, uint32_t
     PCPX_CUDA(cudaStreamSynchronize(ix.qstream()));
 }
 
+void sort_pairs_u64(const pcpx_index& ix, uint64_t* keys, uint32_t* vals, uint32_t n, int n_bits,
+                    uint32_t* launches)
+{
+    if (n == 0)
+        return;
+    SortScratch sc;
+    sc.keys_alt.alloc((size_t)n * 8);
+    sc.vals_alt.alloc(n);
+    uint64_t* keys_alt = reinterpret_cast<uint64_t*>(sc.keys_alt.get());
+    bool const alt = sort_pairs<uint64_t>(keys, vals, keys_alt, sc.vals_alt.get(), n, n_bits,
+                                          ix.qstream(), launches, sc);
+    if (alt)
+    {
+        PCPX_CUDA(cudaMemcpyAsync(keys, keys_alt, (size_t)n * 8, cudaMemcpyDeviceToDevice,
+                                  ix.qstream()));
+        PCPX_CUDA(cudaMemcpyAsync(vals, sc.vals_alt.get(), (size_t)n * 4, cudaMemcpyDeviceToDevice,
+                                  ix.qstream()));
+    }
+    PCPX_CUDA(cudaStreamSynchronize(ix.qstream())); // the scratch is freed on return
+}
+
 } // namespace pcpx

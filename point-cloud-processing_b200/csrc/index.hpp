@@ -135,6 +135,11 @@ pcpx_index* build_index(const float* xyz, size_t n, size_t stride_bytes,
 void sort_queries_by_cell(const pcpx_index& ix, const float* d_queries, uint32_t stride_floats,
                           uint32_t nq, uint32_t* d_order);
 
+// Stable LSD radix sort (radix_sort.cuh) of n (key, value) pairs by key bits [0, n_bits), in
+// place, on the calling thread's stream; adds the kernels it launched to *launches.
+void sort_pairs_u64(const pcpx_index& ix, uint64_t* keys, uint32_t* vals, uint32_t n, int n_bits,
+                    uint32_t* launches);
+
 } // namespace pcpx
 
 inline cudaStream_t pcpx_index::qstream() const

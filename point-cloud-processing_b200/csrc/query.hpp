@@ -72,6 +72,24 @@ void launch_gather_rows(const pcpx_index& ix, const QueryBatch& qb, const ShardI
                         const uint32_t* src, uint32_t* dst, uint32_t width);
 // every list of a CSR (offsets: nq + 1 device values) ascending by value, in place
 void launch_sort_lists(const pcpx_index& ix, const uint64_t* offsets, uint32_t nq, uint32_t* idx);
+// Axis-aligned boxes (query_box.cu, box_core.cuh): nb records of 6 floats {min xyz, max xyz},
+// stride_f floats apart, in device memory; bb = a box every indexed point lies in.
+struct BoxBatch
+{
+    const float* boxes;
+    uint32_t stride_f;
+    uint32_t nb;
+    float bb[6];
+};
+// count[b] = size of box b's list; max_count (nullptr or one zeroed word) = the largest
+void launch_box_count(const pcpx_index& ix, const BoxBatch& bx, uint32_t* count,
+                      uint32_t* max_count);
+// every box's list at idx + offsets[b] (total = offsets[nb]); returns the kernels launched
+uint32_t launch_box_fill(const pcpx_index& ix, const BoxBatch& bx, const uint64_t* offsets,
+                         uint64_t total, uint32_t* idx);
+// every list ascending (PCPX_RADIUS_SORTED); max_count = the longest; returns the kernels launched
+uint32_t launch_box_sort(const pcpx_index& ix, const uint64_t* offsets, uint32_t nb,
+                         uint64_t total, uint32_t max_count, uint32_t* idx);
 void launch_density_keep(const pcpx_index& ix, float r, uint32_t threshold, uint8_t* keep);
 // exclusive scan of `in` (n values) into `out` (n + 1 values, out[n] = total); 64-bit sums
 void launch_exclusive_scan_u32(const pcpx_index& ix, const uint32_t* in, uint32_t n, uint64_t* out);
