@@ -367,6 +367,36 @@ int pcpx_density_filter(
     float* out_xyz,
     size_t* out_n);
 
+/*
+ * Density-based clustering (DBSCAN) of the indexed points, a pcpx extension: the reference has
+ * no clustering.  With min_points <= 1 it is Euclidean clustering, the connected components of
+ * the radius graph.
+ *   - N(p) is exactly the ball pcpx_radius_search returns for p with queries = the cloud: the
+ *     indexed q with fl(d2(p, q)) <= fl(radius * radius), d2 computed without FMA, p included.
+ *     d2 is symmetric bit for bit (negating dx does not change dx * dx), so q in N(p) <=> p in
+ *     N(q).
+ *   - p is core iff |N(p)| >= min_points: exactly the points pcpx_density_filter(radius,
+ *     min_points) keeps.  With min_points 0 or 1 every indexed point is core.
+ *   - clusters are the connected components of the graph on the core points with an edge p - q
+ *     iff q in N(p), numbered 0 .. C-1 in ascending order of the smallest original index among
+ *     their core points (the order of scipy.sparse.csgraph.connected_components).
+ *   - a non-core point with a core point in N(p) takes the label of the core q in N(p) with the
+ *     smallest (fl(d2), original index); every other point is PCPX_NOISE, including the points a
+ *     voxel grid left out of the index.
+ * The labels are unique under these rules: identical bytes whatever the scheduling, for host or
+ * device output, one or several replicas and concurrent calls.
+ * out_labels: n_input entries, host or device.  *out_n_clusters (host, may be NULL) = C.  A NaN
+ * radius is PCPX_ERR_INVALID_ARG; every other radius means what it means for
+ * pcpx_radius_search.  Runs on the primary device of a multi-device index.
+ */
+#define PCPX_NOISE 0xFFFFFFFFu
+int pcpx_cluster_by_density(
+    const pcpx_index* index,
+    float radius,
+    uint32_t min_points,
+    uint32_t* out_labels,
+    uint64_t* out_n_clusters);
+
 /* ---- radius-search callers: smoothing and resampling (SURVEY.md 8f rank 3) ---------------- */
 
 /*

@@ -1353,6 +1353,28 @@ std::vector<typename Index::element_type> filter_by_density(Index const& index, 
     return out;
 }
 
+// pcpx extension (the reference has no clustering): DBSCAN of the indexed elements over the
+// exact ball of `radius` (pcpx_cluster_by_density).  Returns one label per element, in element
+// order: the cluster, numbered 0 .. C-1 in ascending order of each cluster's smallest core
+// element index, or PCPX_NOISE.  An element is core iff filter_by_density(radius, min_points)
+// keeps it; with min_points <= 1 this is Euclidean clustering.  `n_clusters` receives C.
+template <class Index>
+std::vector<std::uint32_t> cluster_by_density(Index const& index, float radius,
+                                              std::size_t min_points,
+                                              std::size_t* n_clusters = nullptr)
+{
+    std::vector<std::uint32_t> labels(index.elements().size());
+    std::uint64_t c = 0;
+    // (a ball holds fewer than 2^32 elements: every larger threshold means no element is core)
+    auto const threshold = static_cast<std::uint32_t>(
+        std::min<std::size_t>(min_points, std::numeric_limits<std::uint32_t>::max()));
+    detail::check(pcpx_cluster_by_density(index.handle(), radius, threshold, labels.data(), &c),
+                  "pcpx_cluster_by_density");
+    if (n_clusters)
+        *n_clusters = static_cast<std::size_t>(c);
+    return labels;
+}
+
 // ---- radius-search callers (SURVEY.md 8f rank 3) ---------------------------------------------
 namespace bilateral {
 // algorithm/bilateral_filter.hpp:28-33

@@ -13,6 +13,7 @@ checked), but every compute call fails loudly when the library or a CUDA device 
 from .capi import (  # noqa: F401
     LIB_PATH,
     NO_NEIGHBOUR,
+    NOISE,
     Index,
     PcpxError,
     bilateral_filter_normals,

@@ -10,6 +10,7 @@ LIB_PATH = os.environ.get("PCPX_LIB", os.path.join(HERE, "lib", "libpcpx.so"))  
 if os.environ.get("PCPX_LIB"):  # an experimental build next to the product (build.py --out=...)
     LIB_PATH = os.environ["PCPX_LIB"]
 NO_NEIGHBOUR = 0xFFFFFFFF
+NOISE = 0xFFFFFFFF  # PCPX_NOISE: the label of a point in no cluster
 
 
 class PcpxError(RuntimeError):
@@ -97,6 +98,8 @@ _SIGNATURES = {
                                          C.POINTER(C.c_double)]),
     "pcpx_density_filter": (C.c_int, [C.c_void_p, C.c_float, C.c_uint32, C.c_void_p, C.c_void_p,
                                       C.POINTER(C.c_size_t)]),
+    "pcpx_cluster_by_density": (C.c_int, [C.c_void_p, C.c_float, C.c_uint32, C.c_void_p,
+                                          C.POINTER(C.c_uint64)]),
     "pcpx_bilateral_filter_points": (C.c_int, [C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p,
                                                C.c_size_t, C.c_double, C.c_double, C.c_uint32,
                                                C.c_int, C.c_void_p, C.POINTER(C.c_float)]),
@@ -518,6 +521,19 @@ class Index:
         if out_xyz is not None and not _is_torch(out_xyz):
             out_xyz = out_xyz[: kept.value]
         return out_mask, out_xyz, kept.value
+
+    def cluster_by_density(self, radius, min_points, out_labels=None):
+        """DBSCAN over the exact ball of radius_search: (labels, n_clusters).  labels[i] is the
+        cluster of point i, 0 .. n_clusters - 1 in ascending order of each cluster's smallest core
+        index, or NOISE.  out_labels: n entries, a numpy uint32 array or a CUDA
+        tensor of 32-bit integers (a new numpy array when None)."""
+        if out_labels is None:
+            out_labels = np.zeros(self.n, np.uint32)
+        bl = _Buf(out_labels, np.uint32, True)
+        nc = C.c_uint64()
+        _check(lib().pcpx_cluster_by_density(self._h, float(radius), int(min_points), bl.ptr,
+                                             C.byref(nc)))
+        return out_labels, nc.value
 
     def orient_normals(self, normals, k, eps=1e-5, nearest_first=False, want_stats=False):
         """propagate_normal_orientations over the kNN graph; `normals` (numpy array or CUDA

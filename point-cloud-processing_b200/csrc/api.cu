@@ -855,6 +855,38 @@ int pcpx_density_filter(const pcpx_index* index, float radius, uint32_t threshol
     });
 }
 
+int pcpx_cluster_by_density(const pcpx_index* index, float radius, uint32_t min_points,
+                            uint32_t* out_labels, uint64_t* out_n_clusters)
+{
+    return guarded([&] {
+        pcpx_index& ix = checked(index);
+        if (std::isnan(radius))
+            fail(PCPX_ERR_INVALID_ARG, "radius is NaN");
+        if (out_n_clusters)
+            *out_n_clusters = 0;
+        size_t const n = ix.n_input;
+        if (n == 0)
+            return;
+        if (!out_labels)
+            fail(PCPX_ERR_INVALID_ARG, "out_labels is NULL");
+        ScopedDevice guard(ix.device);
+        CallStream call(ix); // own stream: calls on one index may run concurrently
+        CallTimer timer(ix);
+        OutBuf<uint32_t> labels;
+        labels.prepare(out_labels, n);
+        uint32_t launches = 0;
+        timer.kernel_begin();
+        uint64_t const n_clusters = launch_cluster_by_density(ix, radius, min_points, labels.d,
+                                                              &launches);
+        timer.kernel_end();
+        ix.timings.kernel_launches = launches;
+        labels.finish(ix.qstream());
+        timer.done();
+        if (out_n_clusters)
+            *out_n_clusters = n_clusters;
+    });
+}
+
 int pcpx_last_timings(const pcpx_index* index, pcpx_timings* out)
 {
     return guarded([&] {

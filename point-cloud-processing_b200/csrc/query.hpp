@@ -91,6 +91,10 @@ uint32_t launch_box_fill(const pcpx_index& ix, const BoxBatch& bx, const uint64_
 uint32_t launch_box_sort(const pcpx_index& ix, const uint64_t* offsets, uint32_t nb,
                          uint64_t total, uint32_t max_count, uint32_t* idx);
 void launch_density_keep(const pcpx_index& ix, float r, uint32_t threshold, uint8_t* keep);
+// DBSCAN labels (cluster.cu): labels = n_input device entries, at original positions; returns the
+// number of clusters and sets *launches to the kernels launched.  Synchronises the stream.
+uint64_t launch_cluster_by_density(const pcpx_index& ix, float r, uint32_t min_points,
+                                   uint32_t* labels, uint32_t* launches);
 // exclusive scan of `in` (n values) into `out` (n + 1 values, out[n] = total); 64-bit sums
 void launch_exclusive_scan_u32(const pcpx_index& ix, const uint32_t* in, uint32_t n, uint64_t* out);
 void launch_exclusive_scan_u8(const pcpx_index& ix, const uint8_t* in, uint32_t n, uint64_t* out);
