@@ -397,6 +397,103 @@ int pcpx_cluster_by_density(
     uint32_t* out_labels,
     uint64_t* out_n_clusters);
 
+/* ---- rigid registration (a pcpx extension: the reference has none) ------------------------- */
+
+/*
+ * Bounded nearest neighbour of transformed queries: the correspondence search of ICP.
+ *   - transformed query: with a row-major 4x4 rigid `transform` T = [R | t], query i is first
+ *     mapped to y_i, each component computed in fp64 as ((R[a][0]*x + R[a][1]*y) + R[a][2]*z)
+ *     + t[a] without FMA, then rounded once to fp32.  NULL means identity: the query is used as is.
+ *   - out_idx[i] = the indexed point q with the smallest (fl(d2), original index) among those with
+ *     fl(d2(y_i, q)) <= fl(max_distance * max_distance), d2 the no-FMA fp32 distance of
+ *     pcpx_knn; out_d2[i] (may be NULL) = that d2.
+ *   - no such point (also for a query with a non-finite coordinate, and for points a voxel grid
+ *     left out of the index): PCPX_NO_NEIGHBOUR and +inf.
+ *   - so the result equals the row of pcpx_knn(k = 1, eps = 0) whenever that row's d2 passes the
+ *     bound.
+ *   - max_distance must be finite and > 0 (else PCPX_ERR_INVALID_ARG); r > 1 is exact, as for
+ *     pcpx_radius_search.
+ * Host or device buffers, strided queries.  Runs on the primary device of a multi-device index.
+ */
+int pcpx_nearest_within(
+    const pcpx_index* index,
+    const float* queries,
+    size_t nq,
+    size_t query_stride_bytes,
+    const double transform[16] /* may be NULL */,
+    float max_distance,
+    uint32_t* out_idx,
+    float* out_d2 /* may be NULL */);
+
+/*
+ * Iterative closest point: the rigid transform that registers `source` to the indexed target.
+ *   - target_normals: n_input rows in original order (what pcpx_estimate_normals(queries = NULL)
+ *     writes), normal_stride_bytes apart; required for point-to-plane, ignored for
+ *     point-to-point.  The sign of a normal does not matter.  A pair whose target normal has a
+ *     non-finite component is not a correspondence.
+ *   - iteration it, from T_0 = init (NULL = identity):
+ *       1. the pairs (y_i, q_i) are those of pcpx_nearest_within(source, T_it, max_distance);
+ *       2. sums in fp64 about c, the centre of the target's root voxel (pcpx_index_bbox):
+ *          point-to-plane A = sum J^T J, b = sum J^T r with J = [(y - c) x n, n],
+ *          r = (y - q) . n; point-to-point sum (y - c), sum (q - c), sum (y - c)(q - c)^T and
+ *          the count; both sum d2;
+ *       3. fewer than 6 (plane) or 3 (point) pairs: stop, PCPX_ICP_TOO_FEW;
+ *       4. solve on the host in fp64: point-to-plane x = (omega, v) = -A^+ b, A^+ the
+ *          pseudo-inverse of a cyclic-Jacobi eigendecomposition (fixed sweep order) without the
+ *          eigenvalues <= 1e-12 * lambda_max, so a motion the pairs do not constrain (a plane
+ *          sliding in itself) is zero; point-to-point Horn's quaternion method (the same Jacobi
+ *          on the 4x4 matrix), never a reflection;
+ *       5. T_it+1 = (y -> R(omega)(y - c) + c + v) o T_it, R by Rodrigues' formula in fp64;
+ *       6. |omega| <= rotation_tolerance and |v| <= translation_tolerance: stop,
+ *          PCPX_ICP_CONVERGED; after max_iterations updates: PCPX_ICP_MAX_ITERATIONS.
+ *   - out_transform = the last T.  out_result and out_correspondences (ns entries, host or
+ *     device, may be NULL: the original index of every source point's pair, or
+ *     PCPX_NO_NEIGHBOUR) describe that T: one more correspondence pass runs after the loop.
+ *     rmse = sqrt(sum d2 / n_correspondences) in fp64, NaN without pairs; fitness =
+ *     n_correspondences / ns.
+ *   - PCPX_ERR_INVALID_ARG: a NaN, infinite or <= 0 max_distance, an unknown metric,
+ *     point-to-plane without normals, params or out_transform NULL.
+ *   - ns == 0 or an empty index: out_transform = init, 0 correspondences, rmse NaN.
+ *   - the bytes of the transform, the result and the correspondences depend on the inputs alone:
+ *     host or device buffers, strided input, repeated and concurrent calls and multi-device
+ *     handles give the same.  Runs on the primary device.
+ *   - pcpx_last_timings covers the whole call; kernel_launches counts every launch.
+ */
+#define PCPX_ICP_POINT_TO_PLANE 0u
+#define PCPX_ICP_POINT_TO_POINT 1u
+#define PCPX_ICP_CONVERGED 0u
+#define PCPX_ICP_MAX_ITERATIONS 1u
+#define PCPX_ICP_TOO_FEW 2u
+typedef struct pcpx_icp_params
+{
+    uint32_t metric;               /* PCPX_ICP_* */
+    uint32_t max_iterations;       /* 0 = 30 */
+    float max_distance;            /* correspondence bound, required: finite, > 0 */
+    double rotation_tolerance;     /* rad; 0 = 1e-6 */
+    double translation_tolerance;  /* 0 = 1e-6 x the diagonal of the target's root voxel */
+    uint32_t reserved[8];
+} pcpx_icp_params;
+typedef struct pcpx_icp_result
+{
+    uint32_t iterations;        /* updates applied */
+    uint32_t stop_reason;       /* PCPX_ICP_CONVERGED / _MAX_ITERATIONS / _TOO_FEW */
+    uint64_t n_correspondences;
+    double fitness;             /* n_correspondences / ns */
+    double rmse;                /* sqrt(sum d2 / n_correspondences), NaN if none */
+} pcpx_icp_result;
+int pcpx_icp(
+    const pcpx_index* target,
+    const float* target_normals,
+    size_t normal_stride_bytes,
+    const float* source,
+    size_t ns,
+    size_t source_stride_bytes,
+    const pcpx_icp_params* params,
+    const double init[16] /* NULL = identity */,
+    double out_transform[16],
+    pcpx_icp_result* out_result /* may be NULL */,
+    uint32_t* out_correspondences /* ns entries, may be NULL */);
+
 /* ---- radius-search callers: smoothing and resampling (SURVEY.md 8f rank 3) ---------------- */
 
 /*

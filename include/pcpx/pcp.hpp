@@ -1375,6 +1375,77 @@ std::vector<std::uint32_t> cluster_by_density(Index const& index, float radius,
     return labels;
 }
 
+// pcpx extension (the reference has no registration): rigid ICP of a source range against the
+// indexed target (pcpx_icp).  `target_normals`: one normal per target element, in element order
+// (what estimate_normals over the index writes); point-to-plane needs them, point-to-point ignores
+// them.  Coordinates of other scalar types are rounded to fp32.  The parameter and result types
+// are pcp::icp::params_t and pcp::icp::result_t.
+} // namespace algorithm
+namespace icp {
+struct params_t
+{
+    std::uint32_t metric         = PCPX_ICP_POINT_TO_PLANE; // or PCPX_ICP_POINT_TO_POINT
+    std::uint32_t max_iterations = 30;
+    float max_distance           = 0.f; // correspondence bound: required, finite, > 0
+    double rotation_tolerance    = 0.0; // 0 = 1e-6 rad
+    double translation_tolerance = 0.0; // 0 = 1e-6 x the diagonal of the target's root voxel
+    std::array<double, 16> init{1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1};
+};
+struct result_t
+{
+    std::array<double, 16> transform; // row-major 4 x 4: source -> target
+    std::uint32_t iterations;
+    std::uint32_t stop_reason; // PCPX_ICP_CONVERGED / _MAX_ITERATIONS / _TOO_FEW
+    std::uint64_t n_correspondences;
+    double fitness;
+    double rmse;
+};
+} // namespace icp
+namespace algorithm {
+
+template <class Index, class NormalRange, class ForwardIter, class PointMap>
+icp::result_t icp(Index const& target_index, NormalRange const& target_normals,
+                  ForwardIter source_begin, ForwardIter source_end, PointMap const& point_map,
+                  icp::params_t const& params)
+{
+    std::vector<float> src;
+    for (auto it = source_begin; it != source_end; ++it)
+    {
+        auto const& p = point_map(*it);
+        src.push_back(static_cast<float>(p.x()));
+        src.push_back(static_cast<float>(p.y()));
+        src.push_back(static_cast<float>(p.z()));
+    }
+    std::vector<float> nrm;
+    if (params.metric == PCPX_ICP_POINT_TO_PLANE)
+        for (auto const& n : target_normals)
+        {
+            nrm.push_back(static_cast<float>(n.x()));
+            nrm.push_back(static_cast<float>(n.y()));
+            nrm.push_back(static_cast<float>(n.z()));
+        }
+    if (params.metric == PCPX_ICP_POINT_TO_PLANE && nrm.size() != 3 * target_index.elements().size())
+        throw std::invalid_argument("icp: point-to-plane needs one normal per target element");
+    pcpx_icp_params prm{};
+    prm.metric                = params.metric;
+    prm.max_iterations        = params.max_iterations;
+    prm.max_distance          = params.max_distance;
+    prm.rotation_tolerance    = params.rotation_tolerance;
+    prm.translation_tolerance = params.translation_tolerance;
+    icp::result_t out{};
+    pcpx_icp_result res{};
+    detail::check(pcpx_icp(target_index.handle(), nrm.empty() ? nullptr : nrm.data(), 12,
+                           src.data(), src.size() / 3, 12, &prm, params.init.data(),
+                           out.transform.data(), &res, nullptr),
+                  "pcpx_icp");
+    out.iterations        = res.iterations;
+    out.stop_reason       = res.stop_reason;
+    out.n_correspondences = res.n_correspondences;
+    out.fitness           = res.fitness;
+    out.rmse              = res.rmse;
+    return out;
+}
+
 // ---- radius-search callers (SURVEY.md 8f rank 3) ---------------------------------------------
 namespace bilateral {
 // algorithm/bilateral_filter.hpp:28-33

@@ -17,7 +17,7 @@ LIBDIR = os.path.join(HERE, "lib")
 OBJDIR = os.path.join(HERE, "build")
 LIB = os.path.join(LIBDIR, "libpcpx.so")
 UNITS = ["index.cu", "query.cu", "query_normals.cu", "query_mean.cu", "api.cu", "smoothing.cu",
-         "orient.cu", "shard.cu", "query_box.cu", "cluster.cu"]
+         "orient.cu", "shard.cu", "query_box.cu", "cluster.cu", "icp.cu"]
 
 NVCC_FLAGS = [
     "-std=c++17", "-O3",

@@ -64,6 +64,31 @@ class Timings(C.Structure):
     ]
 
 
+class IcpParams(C.Structure):
+    _fields_ = [
+        ("metric", C.c_uint32),
+        ("max_iterations", C.c_uint32),
+        ("max_distance", C.c_float),
+        ("rotation_tolerance", C.c_double),
+        ("translation_tolerance", C.c_double),
+        ("reserved", C.c_uint32 * 8),
+    ]
+
+
+class IcpResult(C.Structure):
+    _fields_ = [
+        ("iterations", C.c_uint32),
+        ("stop_reason", C.c_uint32),
+        ("n_correspondences", C.c_uint64),
+        ("fitness", C.c_double),
+        ("rmse", C.c_double),
+    ]
+
+
+ICP_METRICS = {"point_to_plane": 0, "point_to_point": 1}
+ICP_STOP = {0: "converged", 1: "max_iterations", 2: "too_few"}
+
+
 _SIGNATURES = {
     # name: (restype, argtypes)
     "pcpx_device_count": (C.c_int, []),
@@ -100,6 +125,11 @@ _SIGNATURES = {
                                       C.POINTER(C.c_size_t)]),
     "pcpx_cluster_by_density": (C.c_int, [C.c_void_p, C.c_float, C.c_uint32, C.c_void_p,
                                           C.POINTER(C.c_uint64)]),
+    "pcpx_nearest_within": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_size_t,
+                                      C.c_void_p, C.c_float, C.c_void_p, C.c_void_p]),
+    "pcpx_icp": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_size_t,
+                           C.POINTER(IcpParams), C.c_void_p, C.c_void_p, C.POINTER(IcpResult),
+                           C.c_void_p]),
     "pcpx_bilateral_filter_points": (C.c_int, [C.c_void_p, C.c_size_t, C.c_size_t, C.c_void_p,
                                                C.c_size_t, C.c_double, C.c_double, C.c_uint32,
                                                C.c_int, C.c_void_p, C.POINTER(C.c_float)]),
@@ -191,6 +221,15 @@ def _out_rows(like, n, out):
         import torch
         return torch.empty((n, 3), dtype=torch.float32, device=like.device)
     return np.zeros((n, 3), np.float32)
+
+
+def _out_vec(like, n, dtype):
+    """result vector of n entries of the same kind (numpy / torch) as `like`"""
+    if _is_torch(like):
+        import torch
+        tdt = {np.dtype(np.uint32): torch.int32, np.dtype(np.float32): torch.float32}
+        return torch.empty(n, dtype=tdt[np.dtype(dtype)], device=like.device)
+    return np.zeros(n, dtype)
 
 
 def _bilateral(fn, xyz, normals, sigmaf, sigmag, iterations, device, out):
@@ -534,6 +573,54 @@ class Index:
         _check(lib().pcpx_cluster_by_density(self._h, float(radius), int(min_points), bl.ptr,
                                              C.byref(nc)))
         return out_labels, nc.value
+
+    def nearest_within(self, queries, max_distance, transform=None, out_idx=None, out_d2=None):
+        """Bounded nearest neighbour of every query mapped by the 4 x 4 rigid `transform` (None:
+        the queries as they are): (idx, d2), NO_NEIGHBOUR and +inf where no indexed point lies
+        within max_distance.  Numpy arrays or CUDA tensors (results follow the queries' kind
+        unless out_idx / out_d2 are given)."""
+        nq = _count(queries)
+        q = _Buf(queries, np.float32)
+        tf = None if transform is None else np.ascontiguousarray(transform, np.float64).reshape(16)
+        if out_idx is None:
+            out_idx = _out_vec(queries, nq, np.uint32)
+        if out_d2 is None:
+            out_d2 = _out_vec(queries, nq, np.float32)
+        bi, bd = _Buf(out_idx, np.uint32, True), _Buf(out_d2, np.float32, True)
+        _check(lib().pcpx_nearest_within(self._h, q.ptr, nq, 12,
+                                         None if tf is None else tf.ctypes.data,
+                                         float(max_distance), bi.ptr, bd.ptr))
+        return out_idx, out_d2
+
+    def icp(self, source, max_distance, normals=None, metric="point_to_plane", init=None,
+            max_iterations=30, rotation_tolerance=0, translation_tolerance=0,
+            out_correspondences=None, source_stride_bytes=12, normal_stride_bytes=12):
+        """Rigid registration of `source` to the indexed cloud (pcpx_icp): (T, result).  T is the
+        4 x 4 float64 transform mapping the source onto the target; result holds iterations,
+        stop_reason ("converged", "max_iterations", "too_few"), n_correspondences, fitness and
+        rmse.  `normals`: the target's n x 3 normals (point-to-plane).  Numpy arrays or CUDA
+        tensors; out_correspondences (ns entries) receives every source point's pair."""
+        ns = _count(source) if source_stride_bytes == 12 else (
+            (source.numel() if _is_torch(source) else np.asarray(source).size) * 4
+            // source_stride_bytes)
+        bs, bn = _Buf(source, np.float32), _Buf(normals, np.float32)
+        prm = IcpParams()
+        prm.metric = ICP_METRICS[metric] if isinstance(metric, str) else int(metric)
+        prm.max_iterations = int(max_iterations)
+        prm.max_distance = float(max_distance)
+        prm.rotation_tolerance = float(rotation_tolerance)
+        prm.translation_tolerance = float(translation_tolerance)
+        ti = None if init is None else np.ascontiguousarray(init, np.float64).reshape(16)
+        T = np.zeros((4, 4), np.float64)
+        res = IcpResult()
+        bc = _Buf(out_correspondences, np.uint32, True)
+        _check(lib().pcpx_icp(self._h, bn.ptr, normal_stride_bytes, bs.ptr, ns, source_stride_bytes,
+                              C.byref(prm), None if ti is None else ti.ctypes.data,
+                              T.ctypes.data, C.byref(res), bc.ptr))
+        return T, dict(iterations=res.iterations,
+                       stop_reason=ICP_STOP.get(res.stop_reason, res.stop_reason),
+                       n_correspondences=res.n_correspondences, fitness=res.fitness,
+                       rmse=res.rmse)
 
     def orient_normals(self, normals, k, eps=1e-5, nearest_first=False, want_stats=False):
         """propagate_normal_orientations over the kNN graph; `normals` (numpy array or CUDA

@@ -541,7 +541,7 @@ pcpx_index* build_index(const float* xyz, size_t n, size_t stride_bytes,
 }
 
 void sort_queries_by_cell(const pcpx_index& ix, const float* d_queries, uint32_t stride_floats,
-                          uint32_t nq, uint32_t* d_order)
+                          uint32_t nq, uint32_t* d_order, uint32_t* n_launched)
 {
     // Morton order of the queries' own fine cells: neighbouring threads walk neighbouring cells.
     if (nq == 0)
@@ -562,6 +562,8 @@ void sort_queries_by_cell(const pcpx_index& ix, const float* d_queries, uint32_t
         PCPX_CUDA(cudaMemcpyAsync(d_order, sc.vals_alt.get(), (size_t)nq * 4,
                                   cudaMemcpyDeviceToDevice, ix.qstream()));
     PCPX_CUDA(cudaStreamSynchronize(ix.qstream()));
+    if (n_launched)
+        *n_launched += 1 + launches; // the encode kernel + the sort's
 }
 
 void sort_pairs_u64(const pcpx_index& ix, uint64_t* keys, uint32_t* vals, uint32_t n, int n_bits,

@@ -131,9 +131,10 @@ pcpx_index* build_index(const float* xyz, size_t n, size_t stride_bytes,
                         const pcpx_index_params* params);
 
 // Sort helper exported by index.cu for query batches: fills `order` (device, nq entries) with
-// the query permutation sorted by fine Morton code of the query positions.
+// the query permutation sorted by fine Morton code of the query positions; adds the kernels it
+// launched to *launches when given.
 void sort_queries_by_cell(const pcpx_index& ix, const float* d_queries, uint32_t stride_floats,
-                          uint32_t nq, uint32_t* d_order);
+                          uint32_t nq, uint32_t* d_order, uint32_t* launches = nullptr);
 
 // Stable LSD radix sort (radix_sort.cuh) of n (key, value) pairs by key bits [0, n_bits), in
 // place, on the calling thread's stream; adds the kernels it launched to *launches.
